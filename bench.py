@@ -18,6 +18,7 @@ stack, fused resize+NMS, PAF integral + greedy assignment + assembly, results to
   cpu_baseline  the oracle (Caffe CPU arithmetic, im2col + OpenBLAS sgemm, best host thread count) on one full frame
 `--impl reference` times the same oracle on FULL frames of the same workload (one frame per step).
 Frames are sharded one-per-GPU; the only collective is the init broadcast of the packed weights (NCCL).
+`--dump-outputs DIR` writes what the last timed step computed on rank 0 (seeded inputs: two builds compare output for output).
 """
 import argparse
 import json
@@ -42,6 +43,7 @@ WORKLOADS = {
     "C3": ("COCO_18", 656, 368, 1280, 720, 3, 1.0, 0.15, 3, 72, "C3: COCO 656x368, 3 scales (1.0/0.85/0.70), synthetic 720p stream, W-he random-init weights"),
     "C5": ("COCO_18", 992, 736, 1920, 1080, 4, 1.0, 0.15, 1, 24, "C5 per GPU: COCO 992x736, 4 scales (gap 0.15), synthetic 1080p stream, W-he random-init weights"),
 }
+DUMP_BUDGET = 64 << 20   # bytes written by --dump-outputs at most
 
 
 def parse():
@@ -56,7 +58,32 @@ def parse():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--handles", type=int, default=int(os.environ.get("PE_BENCH_HANDLES", "2")),
                     help="engine handles (worker streams) per GPU that alternate over the steps, as rtpose.bin --engines_per_gpu")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed device-resident steps, write what rank 0's last step computed as DIR/<name>.npy (float32): "
+                         "num_people, joints, peaks and the stride-8 maps (leading frames only beyond %d MB)" % (DUMP_BUDGET >> 20))
+    a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    return a
+
+
+def dump_outputs(path, results, maps, max_people):
+    """What a caller of the timed path receives for the B frames of its last step - results[k] = (num_people, joints, peaks) of
+    frame k (pe_fetch), maps = the stride-8 maps of all B frames (pe_fetch_maps) - as float32 .npy files.  joints are zero-padded
+    to max_people persons; maps are kept whole for as many leading frames as the 64 MB budget allows (all of them for every
+    BASELINE workload)."""
+    B = len(results)
+    out = {"num_people": np.array([n for n, _, _ in results], np.float32),
+           "joints": np.zeros((B, max_people) + results[0][1].shape[1:], np.float32),
+           "peaks": np.stack([p for _, _, p in results]).astype(np.float32)}
+    for k, (n, j, _) in enumerate(results):
+        out["joints"][k, :n] = j
+    per_frame = maps.nbytes // B
+    keep = max(0, min(B, (DUMP_BUDGET - sum(a.nbytes for a in out.values())) // per_frame))
+    out["maps"] = maps[:keep * (maps.shape[0] // B)]
+    os.makedirs(path, exist_ok=True)
+    for name, arr in out.items():
+        np.save(os.path.join(path, name + ".npy"), arr)
 
 
 def peaks_info():
@@ -189,8 +216,10 @@ def run_reference(args, rank, world):
         net.process_frame(frames[i % 4], wl.net_h, wl.net_w, wl.S, wl.start, wl.gap)
     t0 = time.time()
     for i in range(args.steps):
-        net.process_frame(frames[i % 4], wl.net_h, wl.net_w, wl.S, wl.start, wl.gap)
+        cnt, joints, peaks, maps = net.process_frame(frames[i % 4], wl.net_h, wl.net_w, wl.S, wl.start, wl.gap)
     dt = time.time() - t0
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, [(cnt, joints, peaks)], maps, orc.MAX_PEOPLE)
     fps = args.steps / dt
     line = {"metric": wl.metric(), "value": fps, "unit": "frames/s", "n_gpus": args.gpus, "steps": args.steps,
             "warmup": args.warmup, "ms_per_step": 1e3 * dt / args.steps, "higher_is_better": True, "scaling": "weak",
@@ -371,6 +400,9 @@ def main():
     ms_dev = maxreduce(ev0.elapsed_time(ev1))
     launches = sumreduce(sum(e.launch_count() for e in engs) - launches0)
     value = world * B * args.steps / (ms_dev * 1e-3)
+    if args.dump_outputs and rank == 0:
+        last = engs[(args.steps - 1) % NH]
+        dump_outputs(args.dump_outputs, [last.fetch(k) for k in range(B)], last.fetch_maps(B), engine.MAX_PEOPLE)
 
     # ---- (2) end to end through the public call: host frames in, joints out, every step
     for i in range(NH):

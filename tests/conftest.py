@@ -7,6 +7,12 @@ ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
 
+# Before any test loads an OpenBLAS: the oracle's convolutions must run the sgemm kernel the reference's outputs in
+# tests/golden/ref_host.npz were recorded with (test_oracle.py::test_conv_vs_reference_code_same_blas).
+from oracle import refcases  # noqa: E402
+
+refcases.pin_blas_core()
+
 
 def pytest_configure(config):
     config.addinivalue_line("markers", "gpu: needs a real B200 (run by the driver with -m gpu)")

@@ -1,5 +1,5 @@
 """GPU parity of the fused resize + NMS + PAF + greedy + assembly kernels (caffe_rtpose_b200/csrc/post.cu)
-through the C ABI, against the oracle AND against the reference's own CUDA kernels (oracle/_ref).
+through the C ABI, against the oracle (which tests/test_oracle.py pins to the reference's own CUDA kernels).
 Everything here is bit-exact."""
 import os
 
@@ -99,29 +99,3 @@ def test_empty_scene():
     cnt, joints, peaks = eng.fetch(0)
     assert cnt == 0 and not peaks.any() and eng.json(joints) == '{\n"version":0.1,\n"bodies":[\n]\n}\n'
     eng.close()
-
-
-@pytest.mark.parametrize("S", [1, 3])
-def test_reference_cuda_kernels_equal_oracle(S):
-    """Pins the oracle's ImResize/NMS restatement to the reference's OWN kernels (imresize_layer.cu, nms_layer.cu)
-    compiled from /root/reference for sm_100a (oracle/_ref/libref_cpm.so)."""
-    R = orc.ref_cpm()
-    if R is None:
-        pytest.skip("oracle/_ref/libref_cpm.so not built")
-    model, net_w, net_h = engine.COCO_18, 320, 176
-    rng = np.random.default_rng(S)
-    for kind in ("scene", "noise"):
-        if kind == "scene":
-            people = synth.make_people(model, 7, net_w, net_h, seed=S)
-            maps8 = synth.make_maps(model, people, net_w, net_h, num_scales=S, start_scale=1.0, scale_gap=0.15, seed=S)
-        else:
-            maps8 = rng.normal(0, 0.5, (S, 57, net_h // 8, net_w // 8)).astype(np.float32)
-        full = orc.imresize(maps8, net_h, net_w, 1.0, 0.15)
-        rfull = np.zeros_like(full)
-        assert R.ref_imresize_host(np.ascontiguousarray(maps8), rfull, S, 57, net_h // 8, net_w // 8, net_h, net_w, 1.0, 0.15) == 0
-        assert np.array_equal(rfull, full)
-        for thr in (0.05, 0.5):
-            opk = orc.nms(full, 18, 64, thr)
-            rpk = np.zeros_like(opk)
-            assert R.ref_nms_host(rfull, rpk, 57, net_h, net_w, 18, 64, thr) == 0
-            assert np.array_equal(rpk, opk)

@@ -2,9 +2,10 @@
 does (rtpose.cpp:183, net.cpp:30-280), for every stage count the reference ships (model/mpi/pose_deploy_linevec_{1,2,4}).
 
 CPU part (no GPU): the engine's prototxt reader + plan builder (pe_plan_describe) against tests/golden/netspec_*.json - the
-layer tables tools/gen_netspec_fixture.py parsed from the reference's files - and, when /root/reference is present, against
-the files themselves; error reporting for graphs outside the pose path.  GPU part: a 2-stage MPI net created from its
+layer tables tools/gen_netspec_fixture.py parsed from the reference's files - and against the files themselves (stored gzipped
+under tests/golden/prototxt/); error reporting for graphs outside the pose path.  GPU part: a 2-stage MPI net created from its
 prototxt, conv stack and whole path against the oracle."""
+import gzip
 import json
 import os
 
@@ -15,7 +16,7 @@ from caffe_rtpose_b200 import engine, synth
 from oracle import orc
 
 GOLD = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
-REF = "/root/reference/model"
+REF = os.path.join(GOLD, "prototxt")   # deploy files of the reference's model/ directory
 SPECS = [("coco", engine.COCO_18, 6), ("mpi", engine.MPI_15, 6), ("mpi_1", engine.MPI_15, 1), ("mpi_2", engine.MPI_15, 2), ("mpi_4", engine.MPI_15, 4)]
 
 
@@ -61,19 +62,23 @@ def test_plan_from_prototxt_matches_the_layer_table(name, model, stages, tmp_pat
         assert engine.plan_describe(model=model).split("\nnms")[0] == engine.plan_describe(prototxt=path).split("\nnms")[0]
 
 
-@pytest.mark.skipif(not os.path.isdir(REF), reason="/root/reference only exists in the build container")
-def test_reference_prototxt_files_parse_directly():
+def test_reference_prototxt_files_parse_directly(tmp_path):
+    def ref_file(rel):
+        path = tmp_path / os.path.basename(rel)
+        with gzip.open(os.path.join(REF, rel + ".gz"), "rb") as f:
+            path.write_bytes(f.read())
+        return str(path)
     for rel, name in (("coco/pose_deploy_linevec.prototxt", "coco"), ("mpi/pose_deploy_linevec.prototxt", "mpi"),
                       ("mpi/pose_deploy_linevec_1.prototxt", "mpi_1"), ("mpi/pose_deploy_linevec_2.prototxt", "mpi_2"),
                       ("mpi/pose_deploy_linevec_4.prototxt", "mpi_4")):
         spec = json.load(open(os.path.join(GOLD, "netspec_%s.json" % name)))
-        plan = parse_plan(engine.plan_describe(prototxt=os.path.join(REF, rel)))
+        plan = parse_plan(engine.plan_describe(prototxt=ref_file(rel)))
         assert [c[1] for c in plan["convs"]] == [l["name"] for l in spec["layers"] if l["type"] == "Convolution"]
     # graphs that are not the PAF pose path are refused with the layer named (the reference would need generic Caffe layers)
     with pytest.raises(engine.PoseEngineError, match="Switch"):
-        engine.plan_describe(prototxt=os.path.join(REF, "mpi/pose_deploy_linevec_switch.prototxt"))
+        engine.plan_describe(prototxt=ref_file("mpi/pose_deploy_linevec_switch.prototxt"))
     with pytest.raises(engine.PoseEngineError, match="3 channels"):
-        engine.plan_describe(prototxt=os.path.join(REF, "mpi/pose_deploy_resize.prototxt"))
+        engine.plan_describe(prototxt=ref_file("mpi/pose_deploy_resize.prototxt"))
 
 
 def test_prototxt_syntax_and_errors(tmp_path):
